@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — graphs/sec through the message-passing hot path, forward + backward (BASELINE.json metric).
 
-    python bench.py [--config NAME] [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--config NAME] [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 --config picks the BASELINE.json configuration (default `masking`, the one the metric is quoted on):
 
@@ -21,6 +21,10 @@ one D2H read of the loss per step (issued asynchronously after the step, consume
 `loss_accum += loss.item()` only feeds a log line).  L2 is flushed between timed steps (256 MiB memset outside the per-step
 event pairs).  `--impl reference` times the reference's OWN model.py on the host cores (oracle/reference_runner.py;
 kind "reference"), or the oracle port of it when the reference's sources are not on the box (kind "port").
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step on the resident batches handed its caller:
+DIR/loss.npy (float64) and DIR/grad.<parameter>.npy (float32) for every parameter.  Batches and initial parameters are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import gc
@@ -32,6 +36,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -253,13 +258,12 @@ def run_reference(args, rank):
     if rank != 0:
         return
     heavy = args.config == "bio_supervised"
-    steps = min(args.steps, 6 if heavy else 500)    # bounded sample: ~4 s (bio) / ~0.1 s (chem) per CPU step
     warmup = min(args.warmup, 1 if heavy else 5)
-    r = cpu_run(args.config, steps, warmup)
+    r = cpu_run(args.config, args.steps, warmup)
     line = {"impl": "reference", "metric": metric_name(args.config), "value": r["value"], "unit": "graphs/s", "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": base_config(args.config, args.gpus),
-            "detail": {"steps_timed": steps, "warmup_run": warmup, "per_step_ms": r["per_step_ms"],
+            "detail": {"steps_timed": args.steps, "warmup_run": warmup, "per_step_ms": r["per_step_ms"],
                        "note": "host cores only; rank 0 runs one replica whatever --gpus says (the reference has no data parallelism)"},
             "cpu_baseline": {"value": r["value"], "unit": "graphs/s", "cores": r["cores"], "kind": r["kind"], "sample": r["sample"]},
             "e2e": {"value": r["value"], "unit": "graphs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
@@ -396,7 +400,7 @@ def run_b200(args, rank, world, local_rank):
                     loss_ready[j].synchronize()
                     acc += float(loss_host[j])
             else:
-                train_step(resident[i % len(resident)])
+                loss = train_step(resident[i % len(resident)])
             ev[i][1].record()
         if e2e:
             for i in range(max(args.steps - LAG, 0), args.steps):
@@ -421,10 +425,13 @@ def run_b200(args, rank, world, local_rank):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         else:
             timed.per_rank = None
+        timed.last_loss = loss if args.steps else None
         return float(t.item()), launches, wall, per, acc / max(args.steps, 1)
 
     with ClockSampler(local_rank) as clocks:
         ms_dev, launches, wall_dev, per_dev, _ = timed(False)
+        # copied before the end-to-end pass below recomputes (and so overwrites) the gradients
+        outputs = step_outputs(step, timed.last_loss) if args.dump_outputs and rank == 0 else None
         host_dev = timed.host_issue_ms
         per_rank_dev = timed.per_rank
         ms_e2e, _, wall_e2e, per_e2e, mean_loss = timed(True)
@@ -475,6 +482,28 @@ def run_b200(args, rank, world, local_rank):
                                                   "sample": cpu["sample"], "value_1thread": cpu["value_1thread"]},
     }
     print(json.dumps(line), flush=True)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
+
+
+def step_outputs(step, loss):
+    """What a training step hands its caller: the loss and every parameter's gradient, copied to host memory."""
+    if loss is None:
+        raise SystemExit("--dump-outputs needs at least one timed step")
+    out = {"loss": loss.detach().double().cpu().numpy()}
+    for name, p in step.named_parameters():
+        if p.grad is not None:
+            out["grad." + name] = p.grad.detach().float().cpu().numpy()
+    return out
+
+
+def dump_outputs(directory, outputs, limit=64 << 20):
+    total = sum(a.nbytes for a in outputs.values())
+    if total > limit:
+        raise SystemExit("--dump-outputs: %d bytes of outputs exceed the %d-byte limit" % (total, limit))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def _profile_rows(cabi, fn, steps):
@@ -618,11 +647,15 @@ def main():
     ap.add_argument("--config", default="masking", choices=CONFIG_NAMES)
     ap.add_argument("--precision", default=None, choices=[None, "fp32", "tf32x3"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's loss and gradients to DIR/<name>.npy (B200 arm)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 20 if args.config == "bio_supervised" else 50
     rank, world, local_rank = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the B200 arm's outputs (--impl b200)")
         run_reference(args, rank)
         return
     if args.warmup < 3:

@@ -13,6 +13,7 @@
 #include <cstdlib>
 #include <map>
 #include <mutex>
+#include <vector>
 
 int pgnn_internal_edge_table_bwd2(const float* S, int Q, const float* g, int64_t ldg, int64_t g_off, int64_t n, int C, float* gT,
                                   int64_t ldt, float* gT2, int q_split, cudaStream_t st);
@@ -45,7 +46,9 @@ int pgnn_internal_bn_apply_fold(const float* x, int64_t ldx, int64_t M, int64_t 
                                 int64_t ldy, cudaStream_t st);
 int pgnn_internal_bn_bwd_colsum(const float* gy, int64_t ldgy, const float* x, int64_t ldx, int64_t M, int64_t C, const float* gamma,
                                 const float* beta, const float* save_mean, const float* save_invstd, int relu, float* gx,
-                                int64_t ldgx, float* ggamma, float* gbeta, float* colsum, void* workspace, cudaStream_t st);
+                                int64_t ldgx, float* ggamma, float* gbeta, float* colsum_part, int* parts, void* workspace, cudaStream_t st);
+int64_t pgnn_internal_bn_colsum_parts(int64_t M);
+int pgnn_internal_fold_colsums(const float* const* part, const int* parts, float* const* out, int count, int64_t C, cudaStream_t st);
 
 namespace {
 
@@ -79,6 +82,8 @@ struct Ws {
   float *gh, *gz2, *gz1, *gaggr;                   // backward temporaries
   float* wT;                                       // [L][2][2D*D]: mlp.0.weight^T, mlp.2.weight^T (dgrad B operands)
   float* wpart;                                    // split-K partial tiles of one wgrad
+  float* bn_part;                                  // [L][bn_parts][D] row-block partials of the mlp.2.bias gradients
+  int64_t bn_parts;
   int64_t wpart_floats;
   void* scratch;                                   // bucket / BatchNorm scratch
   int64_t scratch_bytes, total;
@@ -118,6 +123,8 @@ Ws carve(void* base, int64_t N, int64_t E, int64_t L, int64_t D) {
     if (e > w.wpart_floats) w.wpart_floats = e;
   }
   w.wpart = c.take<float>(w.wpart_floats);
+  w.bn_parts = pgnn_internal_bn_colsum_parts(N);
+  w.bn_part = c.take<float>(L * w.bn_parts * D);
   int64_t sb = pgnn_graph_prep_workspace_bytes(N, E);
   const int64_t bb = pgnn_bn_workspace_bytes(N > 0 ? N : 1, D);
   if (bb > sb) sb = bb;
@@ -353,6 +360,9 @@ int pgnn_chem_gin_backward(const void* const* params, const float* g_node_rep, i
   int64_t ldgy = ldg;
   SideCtx* sc = precision == 1 ? side_ctx(st) : nullptr;
   cudaStream_t wst = sc ? sc->side : st;   // the stream of the weight-gradient GEMMs
+  std::vector<const float*> b2_part;   // mlp.2.bias gradients: row-block partials, folded in block order after the loop
+  std::vector<int> b2_parts;
+  std::vector<float*> b2_out;
   for (int64_t l = L - 1; l >= 0; --l) {
     const void* const* p = params + P_LAYER0 + l * L_COUNT;
     const int64_t* o = off + P_LAYER0 + l * L_COUNT;
@@ -365,9 +375,13 @@ int pgnn_chem_gin_backward(const void* const* params, const float* g_node_rep, i
     float* gz1 = w.gz1 + (sc ? par * N * 2 * D : 0);
     // BatchNorm (+ReLU mask recomputed from z2) backward; the same pass leaves colsum(gz2) = gradient of mlp.2.bias
     if (sc) PGNN_CUDA(cudaStreamWaitEvent(st, sc->w2_done[par], 0));  // layer l+2's wgrad2 has finished reading this copy
+    float* b2p = w.bn_part + l * w.bn_parts * D;
+    int b2n = 0;
     TRY(pgnn_internal_bn_bwd_colsum(gy, ldgy, z2, D, N, D, (const float*)p[L_GAMMA], (const float*)p[L_BETA], w.mean + l * D,
-                                    w.invstd + l * D, !last, gz2, D, grads + o[L_GAMMA], grads + o[L_BETA], grads + o[L_B2],
-                                    w.scratch, st));
+                                    w.invstd + l * D, !last, gz2, D, grads + o[L_GAMMA], grads + o[L_BETA], b2p, &b2n, w.scratch, st));
+    b2_part.push_back(b2p);
+    b2_parts.push_back(b2n);
+    b2_out.push_back(grads + o[L_B2]);
     // MLP backward.  On the tensor path the dgrad epilogues carry the column reductions that would otherwise be
     // passes of their own: colsum(gz1) = gradient of mlp.0.bias, and S^T gaggr = gradient of the two bond tables.
     bool fused = false;
@@ -432,6 +446,7 @@ int pgnn_chem_gin_backward(const void* const* params, const float* g_node_rep, i
     PGNN_CUDA(cudaEventRecord(sc->join, wst));
     PGNN_CUDA(cudaStreamWaitEvent(st, sc->join, 0));
   }
+  TRY(pgnn_internal_fold_colsums(b2_part.data(), b2_parts.data(), b2_out.data(), (int)b2_out.size(), D, st));
   // embedding tables: [120 + 3, D] = onehot^T . gh as a split-K weight-gradient GEMM (the two tables are adjacent in the flat
   // layout); the vector-atomics kernel remains the fallback (FFMA precision, TMA unavailable)
   int rc_e = PGNN_EUNSUPPORTED;

@@ -190,7 +190,7 @@ __global__ void __launch_bounds__(256)
 k_bn_bwd_apply_colsum(const float* __restrict__ gy, int64_t ldgy, const float* __restrict__ x, int64_t ldx, int M, int C,
                       const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ mean,
                       const float* __restrict__ invstd, int relu, const double* __restrict__ sums, float* __restrict__ ggamma,
-                      float* __restrict__ gbeta, float* __restrict__ gx, int64_t ldgx, float* __restrict__ colsum) {
+                      float* __restrict__ gbeta, float* __restrict__ gx, int64_t ldgx, float* __restrict__ colsum_part) {
   pdl_prologue();
   __shared__ float red[8][33];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -221,7 +221,7 @@ k_bn_bwd_apply_colsum(const float* __restrict__ gy, int64_t ldgy, const float* _
     float t = 0.f;
 #pragma unroll
     for (int k = 0; k < 8; ++k) t += red[k][lane];
-    atomicAdd(&colsum[c], t);
+    colsum_part[(int64_t)blockIdx.y * C + c] = t;
   }
 }
 
@@ -279,7 +279,7 @@ __global__ void __launch_bounds__(256)
 k_bn_bwd_apply_colsum_v4(const float* __restrict__ gy, int64_t ldgy, const float* __restrict__ x, int64_t ldx, int M, int C,
                          const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ mean,
                          const float* __restrict__ invstd, int relu, const double* __restrict__ sums, float* __restrict__ ggamma,
-                         float* __restrict__ gbeta, float* __restrict__ gx, int64_t ldgx, float* __restrict__ colsum) {
+                         float* __restrict__ gbeta, float* __restrict__ gx, int64_t ldgx, float* __restrict__ colsum_part) {
   pdl_prologue();
   __shared__ float red[8][128];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -320,11 +320,11 @@ k_bn_bwd_apply_colsum_v4(const float* __restrict__ gy, int64_t ldgy, const float
 #pragma unroll
   for (int q = 0; q < 4; ++q) red[w][lane * 4 + q] = acc[q];
   __syncthreads();
-  if (colsum && threadIdx.x < 128 && blockIdx.x * 128 + threadIdx.x < C) {
+  if (colsum_part && threadIdx.x < 128 && blockIdx.x * 128 + threadIdx.x < C) {
     float t = 0.f;
 #pragma unroll
     for (int k = 0; k < 8; ++k) t += red[k][threadIdx.x];
-    atomicAdd(&colsum[blockIdx.x * 128 + threadIdx.x], t);
+    colsum_part[(int64_t)blockIdx.y * C + blockIdx.x * 128 + threadIdx.x] = t;
   }
 }
 
@@ -488,15 +488,18 @@ int pgnn_internal_bn_apply_fold(const float* x, int64_t ldx, int64_t M, int64_t 
   return PGNN_OK;
 }
 
-// encoder.cu: pgnn_bn_bwd that also leaves the column sums of gx in colsum[C] (OVERWRITTEN)
+// Row blocks of the BatchNorm-backward sweeps below (either variant) for M rows: the size of colsum_part is this x C floats.
+int64_t pgnn_internal_bn_colsum_parts(int64_t M) { return ceil_div(M > 0 ? M : 1, (int64_t)(kVecRows < kStatRows ? kVecRows : kStatRows)); }
+
+// encoder.cu: pgnn_bn_bwd that also leaves the column sums of gx, per row block, in colsum_part[*parts][C]; the caller folds
+// them in block order (pgnn_internal_fold_colsums).  The column sum is the gradient of the bias in front of the BatchNorm:
+// zero in exact arithmetic, so what is computed is cancellation noise, which a fixed summation order keeps the same from run
+// to run (atomics in arrival order did not).
 int pgnn_internal_bn_bwd_colsum(const float* gy, int64_t ldgy, const float* x, int64_t ldx, int64_t M, int64_t C, const float* gamma,
                                 const float* beta, const float* save_mean, const float* save_invstd, int relu, float* gx,
-                                int64_t ldgx, float* ggamma, float* gbeta, float* colsum, void* workspace, cudaStream_t st) {
+                                int64_t ldgx, float* ggamma, float* gbeta, float* colsum_part, int* parts, void* workspace, cudaStream_t st) {
   double* acc = reinterpret_cast<double*>(workspace);
-  float* c1 = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + align_up(2 * C * 8, 256));
-  float* c2 = c1 + C;
   PGNN_CUDA(cudaMemsetAsync(acc, 0, sizeof(double) * 2 * C, st));
-  PGNN_CUDA(cudaMemsetAsync(colsum, 0, sizeof(float) * C, st));
   auto a16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
   if (bn_v4_enabled() && C % 4 == 0 && ldgy % 4 == 0 && ldx % 4 == 0 && ldgx % 4 == 0 && a16(gy) && a16(x) && a16(gx) && a16(gamma) && a16(beta) &&
       a16(save_mean) && a16(save_invstd)) {
@@ -504,16 +507,53 @@ int pgnn_internal_bn_bwd_colsum(const float* gy, int64_t ldgy, const float* x, i
     PGNN_CUDA(pgnn_launch(k_bn_bwd_stats_v4, dim3(gv), dim3(256), 0, st, gy, ldgy, x, ldx, (int)M, (int)C, gamma, beta, save_mean, save_invstd, relu, acc));
     PGNN_LAUNCH_CHECK();
     PGNN_CUDA(pgnn_launch(k_bn_bwd_apply_colsum_v4, dim3(gv), dim3(256), 0, st, gy, ldgy, x, ldx, (int)M, (int)C, gamma, beta, save_mean, save_invstd,
-                          relu, (const double*)acc, ggamma, gbeta, gx, ldgx, colsum));
+                          relu, (const double*)acc, ggamma, gbeta, gx, ldgx, colsum_part));
     PGNN_LAUNCH_CHECK();
+    *parts = (int)gv.y;
     return PGNN_OK;
   }
   dim3 g1((unsigned)ceil_div(C, 32), (unsigned)ceil_div(M, kStatRows));
   PGNN_CUDA(pgnn_launch(k_bn_bwd_stats, dim3(g1), dim3(256), 0, st, gy, ldgy, x, ldx, (int)M, (int)C, gamma, beta, save_mean, save_invstd, relu, acc));
   PGNN_LAUNCH_CHECK();
   PGNN_CUDA(pgnn_launch(k_bn_bwd_apply_colsum, dim3(g1), dim3(256), 0, st, gy, ldgy, x, ldx, (int)M, (int)C, gamma, beta, save_mean, save_invstd, relu,
-                        (const double*)acc, ggamma, gbeta, gx, ldgx, colsum));
+                        (const double*)acc, ggamma, gbeta, gx, ldgx, colsum_part));
   PGNN_LAUNCH_CHECK();
+  *parts = (int)g1.y;
+  return PGNN_OK;
+}
+
+namespace {
+constexpr int kMaxFoldJobs = 16;
+struct ColsumFolds {
+  const float* part[kMaxFoldJobs];
+  float* out[kMaxFoldJobs];
+  int parts[kMaxFoldJobs];
+};
+// out[j][c] = sum over b = 0, 1, ... of part[j][b][c]; blockIdx.y = job
+__global__ void __launch_bounds__(256) k_fold_colsums(ColsumFolds f, int C) {
+  pdl_prologue();
+  const int j = blockIdx.y;
+  for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < C; c += gridDim.x * blockDim.x) {
+    float a = 0.f;
+    for (int b = 0; b < f.parts[j]; ++b) a += f.part[j][(int64_t)b * C + c];
+    f.out[j][c] = a;
+  }
+}
+}  // namespace
+
+// folds the row-block partials of `count` pgnn_internal_bn_bwd_colsum calls (all with C columns), one launch per 16
+int pgnn_internal_fold_colsums(const float* const* part, const int* parts, float* const* out, int count, int64_t C, cudaStream_t st) {
+  for (int first = 0; first < count; first += kMaxFoldJobs) {
+    ColsumFolds f;
+    const int k = count - first < kMaxFoldJobs ? count - first : kMaxFoldJobs;
+    for (int i = 0; i < k; ++i) {
+      f.part[i] = part[first + i];
+      f.out[i] = out[first + i];
+      f.parts[i] = parts[first + i];
+    }
+    PGNN_CUDA(pgnn_launch(k_fold_colsums, dim3((unsigned)ceil_div(C, 256), (unsigned)k), dim3(256), 0, st, f, (int)C));
+    PGNN_LAUNCH_CHECK();
+  }
   return PGNN_OK;
 }
 

@@ -41,9 +41,10 @@ def pretrained_batch(name):
 
 
 def pretrained_state_dict(name):
-    """The checkpoint of PRETRAINED[name]: from /root/reference in the build container, from the staged copy on the GPU box."""
+    """The checkpoint of PRETRAINED[name]: from the reference's tree, or from the copy build() staged from it under oracle/_ref."""
+    from oracle import reference_runner as R
     c = PRETRAINED[name]
-    for root in ("/root/reference", os.path.join(os.path.dirname(HERE), "oracle", "_ref", "weights")):
+    for root in (R.REF_SRC, os.path.join(R.REF_STAGED, "weights")):
         path = os.path.join(root, c["file"])
         if os.path.isfile(path):
             return torch.load(path, map_location="cpu", weights_only=True), path
@@ -52,6 +53,81 @@ def pretrained_state_dict(name):
 
 def golden_params(domain, t):
     return O.make_params(domain, t, 5, 300, seed=CASES[domain]["param_seed"])
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# Stored results of the reference's own code on the inputs of tests/test_oracle_vs_reference.py
+# (tests/golden/make_golden_reference.py).  Full tensors would take megabytes, so exact results are kept as digests and
+# float results as summaries that still carry the element-wise bound the tests state.
+# ---------------------------------------------------------------------------------------------------------------------
+REFERENCE_CHECKS = os.path.join(HERE, "golden", "reference_checks.npz")
+SUMMARY_PROBE_SEED = 12345
+
+
+SUMMARY_K = 20      # elements kept by summary() for gradients and BatchNorm statistics
+
+
+def reference_checks():
+    """name -> stored array.  Gradient and statistics summaries and the digests are stored as two tables (names + rows):
+    every npz member costs a few hundred bytes of headers."""
+    G = dict(np.load(REFERENCE_CHECKS))
+    for name, row in zip(G.pop("summaries|names"), G.pop("summaries|rows")):
+        G[str(name)] = row[:3 + min(int(row[0]), SUMMARY_K)]
+    for name, value in zip(G.pop("digests|names"), G.pop("digests|values")):
+        G[str(name)] = value
+    return G
+
+
+def digest(a):
+    """64-bit digest of an array's values and shape, for exact comparisons (as np.array_equal: the dtype does not count)."""
+    import hashlib
+    a = np.ascontiguousarray(np.asarray(a, dtype=np.float64) + 0.0)   # + 0.0: -0.0 and 0.0 compare equal
+    h = hashlib.sha256(repr(a.shape).encode() + a.tobytes()).digest()
+    return np.frombuffer(h[:8], np.int64)[0]
+
+
+def _flat(t):
+    t = t.detach().cpu() if torch.is_tensor(t) else torch.from_numpy(np.asarray(t))
+    return t.reshape(-1).double()
+
+
+def _positions(n, k):
+    return torch.tensor([(j * 2654435761 + 97) % n for j in range(k)] if n > k else list(range(n)), dtype=torch.long)
+
+
+def _unit_probe(n):
+    p = probe((n,), SUMMARY_PROBE_SEED).double()
+    return p / p.norm()
+
+
+def summary(t, k=SUMMARY_K):
+    """float64 [numel, max|t|, <t, p>, t at k fixed positions], p a seeded unit vector over all elements."""
+    t = _flat(t)
+    n = t.numel()
+    if n == 0:
+        return np.zeros(3)
+    head = [float(n), float(t.abs().max()), float(t @ _unit_probe(n))]
+    return np.concatenate([head, t[_positions(n, k)].numpy()])
+
+
+def summary_close(mine, S, atol, rtol):
+    """Does `mine` meet |mine - ref| <= atol + rtol |ref| on what summary(ref) kept?  The kept elements carry that bound
+    itself; the max-norm and the projection carry what it implies for all elements together:
+    |max|mine| - max|ref|| <= max|mine - ref| and |<mine - ref, p>| <= ||mine - ref||_2 <= sqrt(n) max_i (atol + rtol |ref_i|)."""
+    m = _flat(mine)
+    n = int(S[0])
+    if m.numel() != n:
+        return False
+    if n == 0:
+        return True
+    amax, proj, vals = float(S[1]), float(S[2]), torch.from_numpy(np.asarray(S[3:]))
+    bound = atol + rtol * amax
+    if not bool(((m[_positions(n, len(vals))] - vals).abs() <= atol + rtol * vals.abs()).all()):
+        return False
+    if abs(float(m.abs().max()) - amax) > bound:
+        return False
+    mp = float(m @ _unit_probe(n))
+    return abs(mp - proj) <= n ** 0.5 * bound + 1e-13 * (abs(proj) + float(m.norm()))
 
 
 def load(domain, t):

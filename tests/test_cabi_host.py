@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from oracle import gnn_oracle as O
+from oracle import reference_runner as R
 
 cabi = importlib.import_module("pretrain-gnns_b200._cabi")
 
@@ -48,18 +49,19 @@ def test_state_dict_contract(domain, t):
         ("bio", "gin"): 2726100, ("bio", "gcn"): 467100, ("bio", "graphsage"): 467100, ("bio", "gat"): 941100}[(domain, t)]
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/chem/model_gin/masking.pth"), reason="reference tree absent")
+@pytest.mark.skipif(not os.path.exists(os.path.join(R.REF_SRC, "chem", "model_gin", "masking.pth")),
+                    reason="the reference's shipped checkpoints are not available (2-11 MB each: not part of the repository)")
 def test_shipped_checkpoints_load():
     import glob
     chem = importlib.import_module("pretrain-gnns_b200.chem.model")
     bio = importlib.import_module("pretrain-gnns_b200.bio.model")
     n = 0
     for mod, dom in ((chem, "chem"), (bio, "bio")):
-        for f in sorted(glob.glob(f"/root/reference/{dom}/model_gin/*.pth")):
+        for f in sorted(glob.glob(os.path.join(R.REF_SRC, dom, "model_gin", "*.pth"))):
             sd = torch.load(f, map_location="cpu", weights_only=True)
             assert str(mod.GNN(5, 300).load_state_dict(sd)) == "<All keys matched successfully>"
             n += 1
-        for f in sorted(glob.glob(f"/root/reference/{dom}/model_architecture/*.pth")):
+        for f in sorted(glob.glob(os.path.join(R.REF_SRC, dom, "model_architecture", "*.pth"))):
             t = "gcn" if "gcn" in f else "gat" if "gat" in f else "graphsage" if "graphsage" in f else None
             if t is None:
                 continue

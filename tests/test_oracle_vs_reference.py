@@ -1,129 +1,234 @@
-"""CPU: the oracle restatement against the reference's OWN model.py / batch.py executed here (oracle/reference_runner.py:
-/root/reference in the build container, the staged git-ignored copy under oracle/_ref elsewhere; skipped when neither
-exists).  Unlike the frozen goldens this runs on fresh inputs each time it is asked to: symmetric AND one-direction-only
-graphs (the direction convention), every conv type, both domains, heads, and the batch collators."""
+"""CPU: the oracle restatement against the reference's OWN model.py / batch.py / util.py.  What the reference's files compute
+on the inputs built here is stored in tests/golden/reference_checks.npz (tests/golden/make_golden_reference.py runs them
+over the PyG stand-in on exactly these inputs): exact results as digests; float results as golden_util.summary records
+(a few elements, the max-norm and a seeded projection), on which the element-wise bound each test states is checked.  Symmetric AND one-direction-only graphs (the direction convention),
+every conv type, both domains, heads, the batch collators, the masking transforms and the substructure/context extraction."""
+import functools
 import importlib
-import types
 
 import numpy as np
 import pytest
 import torch
 
+from golden_util import digest, reference_checks, summary_close
 from oracle import gnn_oracle as O
-from oracle import reference_runner as R
 from oracle import step_io_oracle as SO
 
 syn = importlib.import_module("pretrain-gnns_b200.synthetic")
-pytestmark = pytest.mark.skipif(not R.available(), reason="reference sources not available (no /root/reference, no oracle/_ref)")
 TYPES = ("gin", "gcn", "graphsage", "gat")
+NO_CONTEXT = -1   # stands for every digest of an extraction that yields no context graph
 
 
-def _ref_step(mod, P, b, t, domain, training, dtype=torch.float32):
-    model = mod.GNN(5, 300, JK="last", drop_ratio=0, gnn_type=t)
-    assert str(model.load_state_dict(P)) == "<All keys matched successfully>"
-    model.to(dtype).train(training)
-    x = b["x"].to(dtype) if b["x"].is_floating_point() else b["x"]
-    ea = b["edge_attr"].to(dtype) if b["edge_attr"].is_floating_point() else b["edge_attr"]
-    return model, model(x, b["edge_index"], ea)
+@functools.lru_cache(maxsize=1)
+def ref():
+    return reference_checks()
 
 
+def ref_prefixed(prefix):
+    return {k[len(prefix):]: v for k, v in ref().items() if k.startswith(prefix)}
+
+
+def assert_digests(prefix, mine):
+    for k, v in mine.items():
+        assert digest(v) == ref()[prefix + k], k
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# inputs (make_golden_reference.py builds the reference's side from these same functions)
+# ---------------------------------------------------------------------------------------------------------------------
 def _batch(domain, directed, seed):
     b = syn.zinc_batch(6, seed) if domain == "chem" else syn.ppi_batch(2, seed, n_lo=30, n_hi=50, num_tasks=8)
     return syn.one_direction_only(b, seed) if directed else b
 
 
-@pytest.mark.parametrize("directed", [False, True])
-@pytest.mark.parametrize("domain", ["chem", "bio"])
-@pytest.mark.parametrize("t", TYPES)
-def test_oracle_equals_reference_fwd_bwd(domain, t, directed):
-    torch.set_num_threads(1)
-    mod = R.load(domain)
-    b = _batch(domain, directed, 31)
-    P = O.make_params(domain, t, 5, 300, seed=8)
-    fwd = O.chem_gnn if domain == "chem" else O.bio_gnn
-    with torch.no_grad():
-        _, ref_eval = _ref_step(mod, P, b, t, domain, False)
-        mine_eval = fwd(P, b["x"], b["edge_index"], b["edge_attr"], 5, t, False)
-    assert torch.allclose(mine_eval, ref_eval, atol=2e-6, rtol=2e-6), (mine_eval - ref_eval).abs().max()
-    # train-mode forward + backward, float64 on both sides: the two formulations must agree to rounding
-    Rm = torch.randn(ref_eval.shape, generator=torch.Generator().manual_seed(3), dtype=torch.float64)
-    model, y = _ref_step(mod, P, b, t, domain, True, torch.float64)
-    (y * Rm).sum().backward()
-    L = O.leaf_params(P, torch.float64)
-    x = b["x"].double() if b["x"].is_floating_point() else b["x"]
-    ea = b["edge_attr"].double() if b["edge_attr"].is_floating_point() else b["edge_attr"]
-    stats = {}
-    y2 = fwd(L, x, b["edge_index"], ea, 5, t, True, stats)
-    (y2 * Rm).sum().backward()
-    assert torch.allclose(y2, y, atol=1e-10, rtol=1e-9)
-    # per-tensor scale; a conv bias in front of BatchNorm has an exactly-zero gradient (pure rounding noise on both sides),
-    # so the scale is floored at 1e-4 of the model's largest gradient
-    gmax = max(float(p.grad.abs().max()) for p in model.parameters())
-    for k, p in model.named_parameters():
-        scale = max(float(p.grad.abs().max()), 1e-4 * gmax)
-        assert float((L[k].grad - p.grad).abs().max()) <= 1e-9 * scale, k
-    sd = model.state_dict()
-    for k, v in stats.items():
-        assert torch.allclose(v.double(), sd[k].double(), atol=1e-12, rtol=1e-10), k
+def fwd_bwd_key(domain, t, directed):
+    return "fwd_bwd:%s_%s_%s:" % (domain, t, "directed" if directed else "symmetric")
 
 
-def test_direction_convention_is_visible_on_one_direction_graphs():
-    """On the reference's symmetric inputs a swapped target/source is invisible for GIN (SURVEY.md 8(c)); on the
-    one-direction-only graphs used by the parity tests it is not — so those tests do pin the convention."""
-    mod = R.load("chem")
-    P = O.make_params("chem", "gin", 5, 300, seed=8)
-    for directed, differs in ((False, False), (True, True)):
-        b = _batch("chem", directed, 31)
-        with torch.no_grad():
-            _, ref = _ref_step(mod, P, b, "gin", "chem", False)
-            flipped = O.chem_gnn(P, b["x"], b["edge_index"].flip(0), b["edge_attr"], 5, "gin", False)
-        assert (not torch.allclose(flipped, ref, atol=1e-3)) == differs
-
-
-def test_graphpred_heads_equal_reference():
-    """chem/model.py:358-369 and bio/model.py:338-347 (mean pooling, centre-node concat, Linear)."""
+def graphpred_inputs():
     g = torch.Generator().manual_seed(5)
+    out = {}
     for domain, T in (("chem", 12), ("bio", 40)):
-        mod = R.load(domain)
         b = _batch(domain, False, 17)
         P = O.make_params(domain, "gin", 5, 300, seed=2)
         full = {"gnn." + k: v for k, v in P.items()}
         width = 300 if domain == "chem" else 600
         full["graph_pred_linear.weight"] = torch.randn(T, width, generator=g) * 0.05
         full["graph_pred_linear.bias"] = torch.randn(T, generator=g) * 0.05
-        model = mod.GNN_graphpred(5, 300, T, JK="last", drop_ratio=0, graph_pooling="mean", gnn_type="gin")
-        assert str(model.load_state_dict(full)) == "<All keys matched successfully>"
-        model.eval()
+        out[domain] = (T, b, full)
+    return out
+
+
+def collate_masking_inputs():
+    graphs = syn.split_graphs(syn.zinc_batch(9, 23))
+    return graphs, [3, 0, 8, 8, 5]
+
+
+def train_body_inputs(config, T=24):
+    from oracle import steps_oracle as S
+    ts = importlib.import_module("pretrain-gnns_b200.train_steps")
+    if config == "bio_supervised":
+        b = {k: v for k, v in syn.ppi_batch(3, 5, n_lo=30, n_hi=50, num_tasks=T).items() if k in ts.BioSupervisedStep.KEYS}
+    elif config == "contextpred":
+        b = {k: v for k, v in syn.substruct_context_batch(8, 5).items() if k in ts.ContextPredStep.KEYS}
+    else:
+        mb = syn.mask_atoms(syn.zinc_batch(8, 5), 5)
+        b = {k: mb[k] for k in ("x", "edge_index", "edge_attr", "masked_atom_indices")} | {"labels": mb["mask_node_label"][:, 0].contiguous()}
+    return b, S.make_params(config, 3, num_tasks=T)
+
+
+def mask_atoms_inputs():
+    b = syn.zinc_batch(7, 41)
+    node_off = b["ptr"].numpy()
+    return b, syn.split_graphs(b), node_off, SO.mask_atom_choice(node_off, 0.15, seed=12345)
+
+
+def substruct_context_inputs():
+    G = 6
+    sub, ctx = syn.zinc_batch(G, 51, n_lo=12, n_hi=22), syn.zinc_batch(G, 52, n_lo=4, n_hi=14, tree_only=True)
+    sg, cg = syn.split_graphs(sub), syn.split_graphs(ctx)
+    rng = np.random.default_rng(3)
+    center = [int(rng.integers(0, len(g[0]))) for g in sg]
+    overlap = [sorted(rng.choice(len(g[0]), size=int(rng.integers(1, min(4, len(g[0])) + 1)), replace=False).tolist()) for g in cg]
+    return G, sg, cg, center, overlap, [4, 1, 1, 5]
+
+
+def bio_graphs(pb, count):
+    """Per-graph (num_nodes, edge_index, edge_attr) of a ppi_batch, edges local to the graph."""
+    ptr = pb["ptr"].numpy()
+    ei, ea = pb["edge_index"].numpy(), pb["edge_attr"].numpy()
+    owner = np.searchsorted(ptr, ei[0], side="right") - 1
+    eptr = np.searchsorted(owner, np.arange(len(ptr)))
+    return [(int(ptr[g + 1] - ptr[g]), ei[:, eptr[g]:eptr[g + 1]] - ptr[g], ea[eptr[g]:eptr[g + 1]]) for g in range(count)], eptr
+
+
+def bio_collate_inputs():
+    graphs, _ = bio_graphs(syn.ppi_batch(5, 9, n_lo=20, n_hi=35, num_tasks=4), 5)
+    return graphs, [0, 3, 1, 0, 2], [2, 0, 4]
+
+
+EXTRACT_CHEM_PARAMS = [(5, 4, 7), (2, 1, 3), (1, 0, 2), (0, 0, 1), (3, 3, 3), (2, 5, 3)]
+
+
+def extract_chem_inputs():
+    """(x, edge_index, edge_attr, root) for every extraction of the chem test."""
+    rng = np.random.default_rng(7)
+    cases = []
+    for x, ei, ea in syn.split_graphs(syn.zinc_batch(10, 61)):
+        for root in {0, len(x) - 1, int(rng.integers(0, len(x)))}:
+            cases.append((x, ei, ea, root))
+    return cases
+
+
+def extract_pairs_batch_inputs():
+    graphs = syn.split_graphs(syn.zinc_batch(8, 71))
+    ids = [3, 0, 7, 7, 2, 5]
+    roots = SO.draw_roots([len(graphs[g][0]) for g in ids], seed=99)
+    tiny = (graphs[1][0][:1], np.zeros((2, 0), np.int64), np.zeros((0, 2), np.int64))   # a one-atom molecule: no context -> dropped
+    graphs = graphs + [tiny]
+    ids, roots = ids[:3] + [8] + ids[3:], np.concatenate([roots[:3], [0], roots[3:]])
+    return graphs, ids, roots
+
+
+def extract_bio_inputs():
+    """(num_nodes, edge_index, edge_attr, l1) for every extraction of the bio test: graphs without isolated nodes
+    (bio/loader.py:119-142 builds the networkx graph from the edges only: an isolated node would not exist in it and the
+    reference raises a KeyError on the overlap map)."""
+    graphs, _ = bio_graphs(syn.ppi_batch(3, 19, n_lo=30, n_hi=45, pairs_per_node=2, num_tasks=4), 3)
+    cases = []
+    for n, e, a in graphs:
+        a = a.copy()
+        a[0:2, 8] = 1   # a masked pair (bio/util.py:100-102): the round trip through networkx drops the bit
+        if len(np.unique(e)) != n:
+            continue
+        for l1 in (1, 2):
+            cases.append((n, e, a, l1))
+    return cases
+
+
+def mask_edges_chem_inputs():
+    b = syn.zinc_batch(9, 43)
+    node_off = b["ptr"].numpy()
+    return b, syn.split_graphs(b), node_off, SO.mask_atom_choice(node_off, 0.15, seed=777)
+
+
+def mask_edges_bio_inputs():
+    pb = syn.ppi_batch(4, 23, n_lo=20, n_hi=35, pairs_per_node=3, num_tasks=4)
+    graphs, eptr = bio_graphs(pb, 4)
+    return graphs, pb["edge_attr"].numpy(), eptr, SO.mask_edge_choice_bio(eptr, 0.15, seed=31)
+
+
+def _canon_edges(ei, ea, nodes):
+    """Edge multiset in ORIGINAL node ids: sorted rows (u, v, attr...)."""
+    rows = [(int(nodes[int(ei[0, j])]), int(nodes[int(ei[1, j])])) + tuple(float(a) for a in np.asarray(ea[j]).ravel()) for j in range(ei.shape[1])]
+    return sorted(rows)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# tests
+# ---------------------------------------------------------------------------------------------------------------------
+@pytest.mark.parametrize("directed", [False, True])
+@pytest.mark.parametrize("domain", ["chem", "bio"])
+@pytest.mark.parametrize("t", TYPES)
+def test_oracle_equals_reference_fwd_bwd(domain, t, directed):
+    torch.set_num_threads(1)
+    key = fwd_bwd_key(domain, t, directed)
+    b = _batch(domain, directed, 31)
+    P = O.make_params(domain, t, 5, 300, seed=8)
+    fwd = O.chem_gnn if domain == "chem" else O.bio_gnn
+    with torch.no_grad():
+        mine_eval = fwd(P, b["x"], b["edge_index"], b["edge_attr"], 5, t, False)
+    assert summary_close(mine_eval, ref()[key + "eval"], 2e-6, 2e-6)
+    # train-mode forward + backward, float64 on both sides: the two formulations must agree to rounding
+    Rm = torch.randn(mine_eval.shape, generator=torch.Generator().manual_seed(3), dtype=torch.float64)
+    L = O.leaf_params(P, torch.float64)
+    x = b["x"].double() if b["x"].is_floating_point() else b["x"]
+    ea = b["edge_attr"].double() if b["edge_attr"].is_floating_point() else b["edge_attr"]
+    stats = {}
+    y2 = fwd(L, x, b["edge_index"], ea, 5, t, True, stats)
+    (y2 * Rm).sum().backward()
+    assert summary_close(y2, ref()[key + "train"], 1e-10, 1e-9)
+    # per-tensor scale; a conv bias in front of BatchNorm has an exactly-zero gradient (pure rounding noise on both sides),
+    # so the scale is floored at 1e-4 of the model's largest gradient
+    grads = ref_prefixed(key + "grad:")
+    assert set(grads) == {k for k, v in L.items() if v.requires_grad}
+    gmax = max(float(S[1]) for S in grads.values())
+    for k, S in grads.items():
+        scale = max(float(S[1]), 1e-4 * gmax)
+        assert summary_close(L[k].grad, S, 1e-9 * scale, 0.0), k
+    for k, v in stats.items():
+        assert summary_close(v, ref()[key + "stat:" + k], 1e-12, 1e-10), k
+
+
+def test_direction_convention_is_visible_on_one_direction_graphs():
+    """On the reference's symmetric inputs a swapped target/source is invisible for GIN (SURVEY.md 8(c)); on the
+    one-direction-only graphs used by the parity tests it is not — so those tests do pin the convention."""
+    P = O.make_params("chem", "gin", 5, 300, seed=8)
+    for directed, differs in ((False, False), (True, True)):
+        b = _batch("chem", directed, 31)
+        with torch.no_grad():
+            flipped = O.chem_gnn(P, b["x"], b["edge_index"].flip(0), b["edge_attr"], 5, "gin", False)
+        assert (not summary_close(flipped, ref()[fwd_bwd_key("chem", "gin", directed) + "eval"], 1e-3, 1e-5)) == differs
+
+
+def test_graphpred_heads_equal_reference():
+    """chem/model.py:358-369 and bio/model.py:338-347 (mean pooling, centre-node concat, Linear)."""
+    for domain, (T, b, full) in graphpred_inputs().items():
         with torch.no_grad():
             if domain == "chem":
-                ref = model(b["x"], b["edge_index"], b["edge_attr"], b["batch"])
                 mine = O.chem_graphpred(full, b["x"], b["edge_index"], b["edge_attr"], b["batch"], b["num_graphs"], 5, "gin", False)
             else:
-                data = types.SimpleNamespace(**{k: b[k] for k in ("x", "edge_index", "edge_attr", "batch", "center_node_idx")})
-                ref = model(data)
                 mine = O.bio_graphpred(full, b["x"], b["edge_index"], b["edge_attr"], b["batch"], b["center_node_idx"], b["num_graphs"], 5, "gin", False)
-        assert torch.allclose(mine, ref, atol=2e-6, rtol=2e-6)
+        assert torch.allclose(mine, torch.from_numpy(ref()["graphpred:" + domain]), atol=2e-6, rtol=2e-6)
 
 
 def test_collate_oracle_equals_reference_batch_masking():
     """oracle/step_io_oracle.collate_chem against BatchMasking.from_data_list itself (chem/batch.py:17-52), fed
-    per-molecule Data objects that carry MaskAtom's extra keys."""
-    batch_mod = R.load("chem", "batch")
-    from torch_geometric.data import Data  # the stand-in (oracle/pyg103_standin)
-    b = syn.zinc_batch(9, 23)
-    graphs = syn.split_graphs(b)
-    ids = [3, 0, 8, 8, 5]
-    datas = []
-    for g in ids:
-        x, ei, ea = graphs[g]
-        datas.append(Data(x=torch.from_numpy(x.copy()), edge_index=torch.from_numpy(ei.copy()), edge_attr=torch.from_numpy(ea.copy()),
-                          masked_atom_indices=torch.tensor([0, x.shape[0] - 1])))
-    ref = batch_mod.BatchMasking.from_data_list(datas)
+    per-molecule Data objects that carry MaskAtom's extra keys (masked atoms: each molecule's first and last)."""
+    graphs, ids = collate_masking_inputs()
     mine = SO.collate_chem(graphs, ids)
-    for k in ("x", "edge_index", "edge_attr", "batch"):
-        assert np.array_equal(mine[k], ref[k].numpy()), k
     exp_masked = np.concatenate([np.array([0, graphs[g][0].shape[0] - 1]) + mine["node_off"][i] for i, g in enumerate(ids)])
-    assert np.array_equal(exp_masked, ref.masked_atom_indices.numpy())
+    assert_digests("collate_masking:", {k: mine[k] for k in ("x", "edge_index", "edge_attr", "batch")} | {"masked_atom_indices": exp_masked})
 
 
 @pytest.mark.parametrize("config", ["masking", "contextpred", "bio_supervised", "gcn", "gat", "graphsage"])
@@ -132,55 +237,34 @@ def test_train_bodies_port_equals_reference(config):
     reference's own modules, at a small batch."""
     from oracle import steps_oracle as S
     torch.set_num_threads(1)
-    ts = importlib.import_module("pretrain-gnns_b200.train_steps")
-    T = 24
-    if config == "bio_supervised":
-        b = {k: v for k, v in syn.ppi_batch(3, 5, n_lo=30, n_hi=50, num_tasks=T).items() if k in ts.BioSupervisedStep.KEYS}
-    elif config == "contextpred":
-        b = {k: v for k, v in syn.substruct_context_batch(8, 5).items() if k in ts.ContextPredStep.KEYS}
-    else:
-        mb = syn.mask_atoms(syn.zinc_batch(8, 5), 5)
-        b = {k: mb[k] for k in ("x", "edge_index", "edge_attr", "masked_atom_indices")} | {"labels": mb["mask_node_label"][:, 0].contiguous()}
-    P = S.make_params(config, 3, num_tasks=T)
-    ref = S.REFERENCE_STEPS[config]() if config != "bio_supervised" else S.ReferenceBioSupervisedStep(T)
-    ref.load(P)
-    loss_ref = ref(b)
+    key = "train_body:%s:" % config
+    b, P = train_body_inputs(config)
     L = O.leaf_params(P)
     loss, _ = S.LOSSES[config](L, b)
     loss.backward()
-    assert abs(float(loss) - float(loss_ref)) <= 1e-6 * max(1.0, abs(float(loss_ref)))
-    named = {name + "." + k: p for name, m in ref.named.items() for k, p in m.named_parameters()}
-    gmax = max(float(p.grad.abs().max()) for p in named.values())
+    loss_ref = float(ref()[key + "loss"])
+    assert abs(float(loss) - loss_ref) <= 1e-6 * max(1.0, abs(loss_ref))
+    grads = ref_prefixed(key + "grad:")
+    assert set(grads) == {k for k, v in L.items() if v.requires_grad}
+    gmax = max(float(Sg[1]) for Sg in grads.values())
     L64 = O.leaf_params(P, torch.float64)
     S.LOSSES[config](L64, b)[0].backward()
-    for k, p in named.items():
+    for k, Sg in grads.items():
         # a bias in front of train-mode BatchNorm has a structurally zero gradient (fp64: ~1e-17): rounding noise on both sides
         zero = float(L64[k].grad.abs().max()) < 1e-9 * gmax
-        scale = gmax if zero else max(float(p.grad.abs().max()), 1e-3 * gmax)
+        scale = gmax if zero else max(float(Sg[1]), 1e-3 * gmax)
         # same arithmetic in a different order (fp32): agreement to a few ulps of the accumulated magnitude
-        assert float((L[k].grad - p.grad).abs().max()) <= 2e-4 * scale, (k, float((L[k].grad - p.grad).abs().max()) / scale)
+        assert summary_close(L[k].grad, Sg, 2e-4 * scale, 0.0), k
 
 
 def test_mask_atoms_oracle_equals_reference_maskatom():
     """oracle/step_io_oracle.mask_atoms against the reference's own MaskAtom.__call__ fed the same atom choice (its
     `masked_atom_indices` debugging argument, chem/util.py:206,225-241) followed by BatchMasking.from_data_list."""
-    util = R.load("chem", "util")
-    batch_mod = R.load("chem", "batch")
-    from torch_geometric.data import Data
-    b = syn.zinc_batch(7, 41)
-    graphs = syn.split_graphs(b)
-    node_off = b["ptr"].numpy()
-    choice = SO.mask_atom_choice(node_off, 0.15, seed=12345)
+    b, graphs, node_off, choice = mask_atoms_inputs()
     assert [len(c) for c in choice] == [int(len(g[0]) * 0.15 + 1) for g in graphs]
-    t = util.MaskAtom(num_atom_type=119, num_edge_type=5, mask_rate=0.15, mask_edge=False)
-    datas = []
-    for (x, ei, ea), local in zip(graphs, choice):
-        d = Data(x=torch.from_numpy(x.copy()), edge_index=torch.from_numpy(ei.copy()), edge_attr=torch.from_numpy(ea.copy()))
-        datas.append(t(d, masked_atom_indices=list(local)))
-    ref = batch_mod.BatchMasking.from_data_list(datas)
     x2, idx, labels, off = SO.mask_atoms(b["x"].numpy(), node_off, 0.15, seed=12345)
-    assert np.array_equal(x2, ref.x.numpy()) and np.array_equal(idx, ref.masked_atom_indices.numpy())
-    assert np.array_equal(labels, ref.mask_node_label.numpy()) and off[-1] == len(idx)
+    assert_digests("mask_atoms:", {"x": x2, "masked_atom_indices": idx, "mask_node_label": labels})
+    assert off[-1] == len(idx)
     # the draw is a uniform k-subset: over many seeds every node of a graph is chosen about equally often
     n0 = int(node_off[1])
     hits = np.zeros(n0)
@@ -192,232 +276,102 @@ def test_mask_atoms_oracle_equals_reference_maskatom():
 
 def test_substruct_context_collate_oracle_equals_reference():
     """chem/batch.py:141-210: BatchSubstructContext.from_data_list on per-pair Data objects vs collate_chem x 2 + collate_lists."""
-    batch_mod = R.load("chem", "batch")
-    from torch_geometric.data import Data
-    G = 6
-    sub, ctx = syn.zinc_batch(G, 51, n_lo=12, n_hi=22), syn.zinc_batch(G, 52, n_lo=4, n_hi=14, tree_only=True)
-    sg, cg = syn.split_graphs(sub), syn.split_graphs(ctx)
-    rng = np.random.default_rng(3)
-    center = [int(rng.integers(0, len(g[0]))) for g in sg]
-    overlap = [sorted(rng.choice(len(g[0]), size=int(rng.integers(1, min(4, len(g[0])) + 1)), replace=False).tolist()) for g in cg]
-    ids = [4, 1, 1, 5]
-    datas = []
-    for g in ids:
-        T = lambda a: torch.from_numpy(np.asarray(a).copy())
-        datas.append(Data(x=T(sg[g][0]), edge_index=T(sg[g][1]), edge_attr=T(sg[g][2]),   # the main graph (unused by the collator but num_nodes reads x)
-                          x_substruct=T(sg[g][0]), edge_index_substruct=T(sg[g][1]), edge_attr_substruct=T(sg[g][2]),
-                          center_substruct_idx=torch.tensor([center[g]]),
-                          x_context=T(cg[g][0]), edge_index_context=T(cg[g][1]), edge_attr_context=T(cg[g][2]),
-                          overlap_context_substruct_idx=torch.tensor(overlap[g])))
-    ref = batch_mod.BatchSubstructContext.from_data_list(datas)
+    G, sg, cg, center, overlap, ids = substruct_context_inputs()
     s, c = SO.collate_chem(sg, ids), SO.collate_chem(cg, ids)
     cptr, optr = np.arange(G + 1), np.cumsum([0] + [len(o) for o in overlap])
     cen, _, _, _ = SO.collate_lists(cptr, np.array(center), ids, add=s["node_off"])
     ov, seg, sizes, _ = SO.collate_lists(optr, np.concatenate(overlap), ids, add=c["node_off"])
-    for k, v in (("x_substruct", s["x"]), ("edge_index_substruct", s["edge_index"]), ("edge_attr_substruct", s["edge_attr"]),
-                 ("center_substruct_idx", cen), ("x_context", c["x"]), ("edge_index_context", c["edge_index"]),
-                 ("edge_attr_context", c["edge_attr"]), ("overlap_context_substruct_idx", ov), ("batch_overlapped_context", seg),
-                 ("overlapped_context_size", sizes)):
-        assert np.array_equal(v, ref[k].numpy()), k
+    assert_digests("substruct_context_collate:", {
+        "x_substruct": s["x"], "edge_index_substruct": s["edge_index"], "edge_attr_substruct": s["edge_attr"], "center_substruct_idx": cen,
+        "x_context": c["x"], "edge_index_context": c["edge_index"], "edge_attr_context": c["edge_attr"],
+        "overlap_context_substruct_idx": ov, "batch_overlapped_context": seg, "overlapped_context_size": sizes})
 
 
 def test_bio_collate_oracle_equals_reference():
     """bio/batch.py:17-50 (BatchFinetune.from_data_list, the collator of bio/dataloader.py's DataLoaderFinetune: edge_index
     and center_node_idx offset by the running node count) vs collate_bio + collate_lists."""
-    batch_mod = R.load("bio", "batch")
-    from torch_geometric.data import Data
-    pb = syn.ppi_batch(5, 9, n_lo=20, n_hi=35, num_tasks=4)
-    ptr = pb["ptr"].numpy()
-    ei, ea = pb["edge_index"].numpy(), pb["edge_attr"].numpy()
-    owner = np.searchsorted(ptr, ei[0], side="right") - 1
-    eptr = np.searchsorted(owner, np.arange(len(ptr)))
-    graphs = [(int(ptr[g + 1] - ptr[g]), ei[:, eptr[g]:eptr[g + 1]] - ptr[g], ea[eptr[g]:eptr[g + 1]]) for g in range(5)]
-    centers = [0, 3, 1, 0, 2]
-    ids = [2, 0, 4]
-    datas = [Data(x=torch.ones(graphs[g][0], 1), edge_index=torch.from_numpy(graphs[g][1].copy()), edge_attr=torch.from_numpy(graphs[g][2].copy()),
-                  center_node_idx=torch.tensor([centers[g]])) for g in ids]
-    ref = batch_mod.BatchFinetune.from_data_list(datas)
+    graphs, centers, ids = bio_collate_inputs()
     mine = SO.collate_bio(graphs, ids)
-    for k in ("x", "edge_index", "edge_attr", "batch"):
-        assert np.array_equal(mine[k], ref[k].numpy()), k
     cen, _, _, _ = SO.collate_lists(np.arange(6), np.array(centers), ids, add=mine["node_off"])
-    assert np.array_equal(cen, ref.center_node_idx.numpy())
+    assert_digests("bio_collate:", {k: mine[k] for k in ("x", "edge_index", "edge_attr", "batch")} | {"center_node_idx": cen})
 
 
-def _canon_edges(ei, ea, nodes):
-    """Edge multiset in ORIGINAL node ids: sorted rows (u, v, attr...)."""
-    rows = [(int(nodes[int(ei[0, j])]), int(nodes[int(ei[1, j])])) + tuple(float(a) for a in np.asarray(ea[j]).ravel()) for j in range(ei.shape[1])]
-    return sorted(rows)
+def pair_digests(nodes_s, nodes_c, canon_s, canon_c, center, overlap):
+    return [digest(v) for v in (nodes_s, nodes_c, canon_s, canon_c, [center], overlap)]
 
 
-def _ref_extract(util, transform, data, root):
-    """Run the reference's ExtractSubstructureContextPair and return its output together with the old->new node maps it
-    built (util.reset_idxes is a module-level function looked up at call time: wrap it to record the maps)."""
-    maps = []
-    orig = util.reset_idxes
-
-    def recording(G):
-        new_G, mapping = orig(G)
-        maps.append(dict(mapping))
-        return new_G, mapping
-
-    util.reset_idxes = recording
-    try:
-        out = transform(data, root_idx=root)
-    finally:
-        util.reset_idxes = orig
-    return out, maps
-
-
-@pytest.mark.parametrize("k,l1,l2", [(5, 4, 7), (2, 1, 3), (1, 0, 2), (0, 0, 1), (3, 3, 3), (2, 5, 3)])
+@pytest.mark.parametrize("k,l1,l2", EXTRACT_CHEM_PARAMS)
 def test_extract_substruct_context_oracle_equals_reference_chem(k, l1, l2):
     """oracle/step_io_oracle.extract_pair against the reference's own ExtractSubstructureContextPair.__call__(data, root_idx)
     (chem/util.py:55-151) on molecules with duplicate bonds (the synthetic generator's extra pairs can repeat one), for the
     script's default (k, l1, l2) = (5, 4, 7) (chem/pretrain_contextpred.py:145-150), small radii, the 0 -> -1 quirk, an
-    empty context (l1 == l2) and l1 > l2.  The reference's node numbering is undone through the maps it built."""
-    util = R.load("chem", "util")
-    from torch_geometric.data import Data
-    b = syn.zinc_batch(10, 61)
-    graphs = syn.split_graphs(b)
-    t = util.ExtractSubstructureContextPair(k, l1, l2)
-    rng = np.random.default_rng(7)
-    for x, ei, ea in graphs:
-        for root in {0, len(x) - 1, int(rng.integers(0, len(x)))}:
-            d = Data(x=torch.from_numpy(x.copy()), edge_index=torch.from_numpy(ei.copy()), edge_attr=torch.from_numpy(ea.copy()))
-            ref, maps = _ref_extract(util, t, d, root)
-            mine = SO.extract_pair(x, ei, ea, root, k, l1, l2)
-            if mine is None:
-                assert not hasattr(ref, "x_context") or ref.x_context is None
-                continue
-            ms, mc = maps[0], maps[1]
-            inv_s = {new: old for old, new in ms.items()}
-            inv_c = {new: old for old, new in mc.items()}
-            assert sorted(ms) == mine["nodes_substruct"].tolist() and sorted(mc) == mine["nodes_context"].tolist()
-            for new, old in inv_s.items():
-                assert np.array_equal(ref.x_substruct[new].numpy(), x[old])
-            for new, old in inv_c.items():
-                assert np.array_equal(ref.x_context[new].numpy(), x[old])
-            assert np.array_equal(mine["x_substruct"], x[mine["nodes_substruct"]]) and np.array_equal(mine["x_context"], x[mine["nodes_context"]])
-            ref_s = _canon_edges(ref.edge_index_substruct.numpy(), ref.edge_attr_substruct.numpy(), inv_s)
-            ref_c = _canon_edges(ref.edge_index_context.numpy(), ref.edge_attr_context.numpy(), inv_c)
-            assert ref_s == _canon_edges(mine["edge_index_substruct"], mine["edge_attr_substruct"], mine["nodes_substruct"])
-            assert ref_c == _canon_edges(mine["edge_index_context"], mine["edge_attr_context"], mine["nodes_context"])
-            assert inv_s[int(ref.center_substruct_idx)] == root == mine["nodes_substruct"][mine["center_substruct_idx"]]
-            ov_ref = sorted(inv_c[int(i)] for i in ref.overlap_context_substruct_idx) if hasattr(ref, "overlap_context_substruct_idx") and \
-                ref.overlap_context_substruct_idx is not None else []
-            assert ov_ref == mine["nodes_context"][mine["overlap_context_substruct_idx"]].tolist()
+    empty context (l1 == l2) and l1 > l2.  Compared in original node ids (the reference's own numbering undone through the
+    maps it built): node sets, edge multisets, centre and overlap nodes."""
+    rows = []
+    for x, ei, ea, root in extract_chem_inputs():
+        mine = SO.extract_pair(x, ei, ea, root, k, l1, l2)
+        if mine is None:
+            rows.append([NO_CONTEXT] * 6)
+            continue
+        ns, nc = mine["nodes_substruct"], mine["nodes_context"]
+        assert np.array_equal(mine["x_substruct"], x[ns]) and np.array_equal(mine["x_context"], x[nc])
+        assert ns[mine["center_substruct_idx"]] == root
+        rows.append(pair_digests(ns.tolist(), nc.tolist(), _canon_edges(mine["edge_index_substruct"], mine["edge_attr_substruct"], ns),
+                                 _canon_edges(mine["edge_index_context"], mine["edge_attr_context"], nc), root,
+                                 nc[mine["overlap_context_substruct_idx"]].tolist()))
+    want = ref()["extract_chem:%d_%d_%d" % (k, l1, l2)]
+    assert want.shape == (len(rows), 6)
+    for i, r in enumerate(rows):
+        assert np.array_equal(np.array(r, np.int64), want[i]), (i, ["nodes_s", "nodes_c", "edges_s", "edges_c", "center", "overlap"])
 
 
 def test_extract_pairs_batch_oracle_equals_reference_collation():
     """extract_pairs_batch = the per-graph extraction followed by BatchSubstructContext.from_data_list (chem/batch.py:141-210),
     including the reference's silent drop of pairs without a context.  The per-graph Data objects handed to the reference's
     collator carry THIS oracle's (canonically ordered) fields, so the comparison is exact."""
-    batch_mod = R.load("chem", "batch")
-    from torch_geometric.data import Data
-    graphs = syn.split_graphs(syn.zinc_batch(8, 71))
-    ids = [3, 0, 7, 7, 2, 5]
-    roots = SO.draw_roots([len(graphs[g][0]) for g in ids], seed=99)
-    tiny = (graphs[1][0][:1], np.zeros((2, 0), np.int64), np.zeros((0, 2), np.int64))   # a one-atom molecule: no context -> dropped
-    graphs = graphs + [tiny]
-    ids, roots = ids[:3] + [8] + ids[3:], np.concatenate([roots[:3], [0], roots[3:]])
-    T = lambda a: torch.from_numpy(np.ascontiguousarray(a))
-    datas = []
-    for g, r in zip(ids, roots):
-        x, ei, ea = graphs[g]
-        p = SO.extract_pair(x, ei, ea, int(r), 2, 1, 3)
-        d = Data(x=T(x), edge_index=T(ei), edge_attr=T(ea))
-        if p is not None:
-            for k_ in ("x_substruct", "edge_index_substruct", "edge_attr_substruct", "x_context", "edge_index_context", "edge_attr_context",
-                       "overlap_context_substruct_idx"):
-                setattr(d, k_, T(p[k_]))
-            d.center_substruct_idx = torch.tensor([p["center_substruct_idx"]])
-        datas.append(d)
-    ref = batch_mod.BatchSubstructContext.from_data_list(datas)
+    graphs, ids, roots = extract_pairs_batch_inputs()
     mine = SO.extract_pairs_batch(graphs, ids, roots, 2, 1, 3)
     assert mine["kept"].tolist() == [0, 1, 2, 4, 5, 6]
-    for k_ in ("x_substruct", "edge_index_substruct", "edge_attr_substruct", "center_substruct_idx", "x_context", "edge_index_context",
-               "edge_attr_context", "overlap_context_substruct_idx", "batch_overlapped_context", "overlapped_context_size"):
-        assert np.array_equal(mine[k_], ref[k_].numpy()), k_
+    assert_digests("extract_pairs_batch:", {k_: mine[k_] for k_ in (
+        "x_substruct", "edge_index_substruct", "edge_attr_substruct", "center_substruct_idx", "x_context", "edge_index_context",
+        "edge_attr_context", "overlap_context_substruct_idx", "batch_overlapped_context", "overlapped_context_size")})
 
 
 def test_extract_context_oracle_equals_reference_bio():
     """bio/util.py:123-205 (substructure = the whole ego graph, context = everything further than l1 hops from the centre,
-    every context node an overlap node) on graphs without isolated nodes (bio/loader.py:119-142 builds the networkx graph
-    from the edges only: an isolated node would not exist in it and the reference raises a KeyError on the overlap map)."""
-    util = R.load("bio", "util")
-    from torch_geometric.data import Data
-    pb = syn.ppi_batch(3, 19, n_lo=30, n_hi=45, pairs_per_node=2, num_tasks=4)
-    ptr = pb["ptr"].numpy()
-    ei, ea = pb["edge_index"].numpy(), pb["edge_attr"].numpy()
-    owner = np.searchsorted(ptr, ei[0], side="right") - 1
-    eptr = np.searchsorted(owner, np.arange(len(ptr)))
-    for g in range(3):
-        n = int(ptr[g + 1] - ptr[g])
-        e, a = ei[:, eptr[g]:eptr[g + 1]] - ptr[g], ea[eptr[g]:eptr[g + 1]].copy()
-        a[0:2, 8] = 1   # a masked pair (bio/util.py:100-102): the round trip through networkx drops the bit
-        if len(np.unique(e)) != n:
+    every context node an overlap node); nx_to_graph_data_obj (bio/loader.py:76-116) re-emits w1..w7 and zeros for the
+    self-loop / mask columns of the context edges."""
+    rows = []
+    for n, e, a, l1 in extract_bio_inputs():
+        mine = SO.extract_pair(np.ones((n, 1), np.float32), e, a, 0, 0, l1, 0, whole_graph=True)
+        if mine is None:
+            rows.append([NO_CONTEXT] * 4)
             continue
-        for l1 in (1, 2):
-            t = util.ExtractSubstructureContextPair(l1, center=True)
-            d = Data(x=torch.ones(n, 1), edge_index=torch.from_numpy(e.copy()), edge_attr=torch.from_numpy(a.copy()), center_node_idx=torch.tensor([0]))
-            ref, maps = _ref_extract(util, t, d, None)
-            mine = SO.extract_pair(np.ones((n, 1), np.float32), e, a, 0, 0, l1, 0, whole_graph=True)
-            if mine is None:
-                assert not hasattr(ref, "x_context") or ref.x_context is None
-                continue
-            inv_c = {new: old for old, new in maps[0].items()}
-            assert sorted(maps[0]) == mine["nodes_context"].tolist()
-            assert tuple(ref.x_context.shape) == mine["x_context"].shape
-            # nx_to_graph_data_obj (bio/loader.py:76-116) re-emits w1..w7 and zeros for the self-loop / mask columns
-            assert _canon_edges(ref.edge_index_context.numpy(), ref.edge_attr_context.numpy(), inv_c) == \
-                _canon_edges(mine["edge_index_context"], mine["edge_attr_context"], mine["nodes_context"])
-            assert sorted(inv_c[int(i)] for i in ref.overlap_context_substruct_idx) == mine["nodes_context"][mine["overlap_context_substruct_idx"]].tolist()
-            assert np.array_equal(ref.edge_index_substruct.numpy(), e) and int(ref.center_substruct_idx) == 0
+        nc = mine["nodes_context"]
+        rows.append([digest(v) for v in (nc.tolist(), list(mine["x_context"].shape), _canon_edges(mine["edge_index_context"], mine["edge_attr_context"], nc),
+                                          nc[mine["overlap_context_substruct_idx"]].tolist())])
+    want = ref()["extract_bio"]
+    assert len(rows) > 0 and want.shape == (len(rows), 4)
+    for i, r in enumerate(rows):
+        assert np.array_equal(np.array(r, np.int64), want[i]), (i, ["nodes_c", "x_context_shape", "edges_c", "overlap"])
 
 
 def test_mask_edges_chem_oracle_equals_reference_maskatom_mask_edge():
     """oracle mask_edges_chem against the reference's MaskAtom(mask_edge=True).__call__(data, masked_atom_indices=choice)
     (chem/util.py:243-272) followed by BatchMasking.from_data_list (chem/batch.py:17-52: connected_edge_indices + cumsum_edge)."""
-    util = R.load("chem", "util")
-    batch_mod = R.load("chem", "batch")
-    from torch_geometric.data import Data
-    b = syn.zinc_batch(9, 43)
-    graphs = syn.split_graphs(b)
-    node_off = b["ptr"].numpy()
-    choice = SO.mask_atom_choice(node_off, 0.15, seed=777)
-    t = util.MaskAtom(num_atom_type=119, num_edge_type=5, mask_rate=0.15, mask_edge=True)
-    datas = []
-    for (x, ei, ea), local in zip(graphs, choice):
-        d = Data(x=torch.from_numpy(x.copy()), edge_index=torch.from_numpy(ei.copy()), edge_attr=torch.from_numpy(ea.copy()))
-        datas.append(t(d, masked_atom_indices=list(local)))
-    ref = batch_mod.BatchMasking.from_data_list(datas)
-    x2, idx, _, _ = SO.mask_atoms(b["x"].numpy(), node_off, 0.15, seed=777)
+    b, graphs, node_off, _ = mask_edges_chem_inputs()
+    _, idx, _, _ = SO.mask_atoms(b["x"].numpy(), node_off, 0.15, seed=777)
     edge_off = np.concatenate([[0], np.cumsum([g[1].shape[1] for g in graphs])])
     ea2, conn, lab, off = SO.mask_edges_chem(b["edge_index"].numpy(), b["edge_attr"].numpy(), edge_off, idx)
-    assert np.array_equal(ea2, ref.edge_attr.numpy()) and np.array_equal(conn, ref.connected_edge_indices.numpy())
-    assert np.array_equal(lab, ref.mask_edge_label.numpy()) and off[-1] == len(conn) and len(conn) > 0
+    assert_digests("mask_edges_chem:", {"edge_attr": ea2, "connected_edge_indices": conn, "mask_edge_label": lab})
+    assert off[-1] == len(conn) and len(conn) > 0
 
 
 def test_mask_edges_bio_oracle_equals_reference_maskedge():
     """oracle mask_edges_bio against the reference's MaskEdge.__call__(data, masked_edge_indices=[2 i ...]) (bio/util.py:46-104)
     followed by bio BatchMasking.from_data_list (bio/batch.py:71-105: masked_edge_idx + cumsum_edge)."""
-    util = R.load("bio", "util")
-    batch_mod = R.load("bio", "batch")
-    from torch_geometric.data import Data
-    pb = syn.ppi_batch(4, 23, n_lo=20, n_hi=35, pairs_per_node=3, num_tasks=4)
-    ptr = pb["ptr"].numpy()
-    ei, ea = pb["edge_index"].numpy(), pb["edge_attr"].numpy()
-    owner = np.searchsorted(ptr, ei[0], side="right") - 1
-    eptr = np.searchsorted(owner, np.arange(len(ptr)))
-    choice = SO.mask_edge_choice_bio(eptr, 0.15, seed=31)
+    _, ea, eptr, choice = mask_edges_bio_inputs()
     assert [len(c) for c in choice] == [int((eptr[g + 1] - eptr[g]) // 2 * 0.15 + 1) for g in range(4)]
-    t = util.MaskEdge(mask_rate=0.15)
-    datas = []
-    for g in range(4):
-        n = int(ptr[g + 1] - ptr[g])
-        d = Data(x=torch.ones(n, 1), edge_index=torch.from_numpy(ei[:, eptr[g]:eptr[g + 1]] - ptr[g]), edge_attr=torch.from_numpy(ea[eptr[g]:eptr[g + 1]].copy()))
-        datas.append(t(d, masked_edge_indices=[2 * i for i in choice[g]]))
-    ref = batch_mod.BatchMasking.from_data_list(datas)
     ea2, idx, lab, off = SO.mask_edges_bio(ea, eptr, 0.15, seed=31)
-    assert np.array_equal(ea2, ref.edge_attr.numpy()) and np.array_equal(idx, ref.masked_edge_idx.numpy())
-    assert np.array_equal(lab, ref.mask_edge_label.numpy()) and off[-1] == len(idx)
+    assert_digests("mask_edges_bio:", {"edge_attr": ea2, "masked_edge_idx": idx, "mask_edge_label": lab})
+    assert off[-1] == len(idx)
